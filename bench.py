@@ -2,15 +2,17 @@
 """bench.py -- BASELINE.json metric: UNet denoising steps/sec @ 768x768, 4 images (UNet batch 8 under CFG),
 Kandinsky-2.2 decoder configuration (1.22 B-parameter UNet, 32 context tokens, guidance 4, DDPM learned-range).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One "step" = one classifier-free-guidance-doubled UNet forward + guidance combine + scheduler update for the
 batch (SURVEY.md 8d).  Own arm: the C-ABI kernels of libk2b200.so replayed as a CUDA graph; one process per
 GPU, each rank denoises its own 4 images (weak scaling, the only collective is one NCCL broadcast of the
 conditioning embeddings before step 0).  `value` times K steps with the latents resident in HBM; `e2e` times
 the same K steps through the module boundary with the latents coming from / returning to pinned host memory
-every step.  `--impl reference` times the reference algorithm's CPU path (the oracle port of the reference
-modules -- /root/reference itself is Python and absent on the GPU box) on the host cores.
+every step.  `--dump-outputs DIR` writes the latents of the last timed step to DIR/latent.npy (float32), so that two
+builds run with the same arguments (hence the same seeded weights, embeddings, noise and latents) can be compared output
+for output.  `--impl reference` times the reference algorithm's CPU path (the oracle port of the reference
+modules; the reference itself is Python and not part of this repository) on the host cores.
 """
 import argparse
 import json
@@ -298,6 +300,28 @@ def step_roofline(plan, ms_per_step, n_unet, H, W, peaks, reps=2):
     }
 
 
+DUMP_LIMIT_BYTES = (64 << 20) - 4096  # 64 MB in all, less room for the .npy header
+
+
+def dump_latent(out_dir, x, world, rank):
+    """--dump-outputs: the latents the timed path returned after its last step, every rank's rows in rank order, as
+    out_dir/latent.npy (float32).  Above the size limit a fixed, seeded sample of the flattened elements is written."""
+    import numpy as np
+    if world > 1:
+        import torch.distributed as dist
+        parts = [torch.empty_like(x) for _ in range(world)]
+        dist.all_gather(parts, x.contiguous())
+        x = torch.cat(parts)
+    if rank != 0:
+        return
+    a = x.float().cpu().numpy()
+    if a.nbytes > DUMP_LIMIT_BYTES:
+        keep = np.random.default_rng(0).choice(a.size, DUMP_LIMIT_BYTES // a.itemsize, replace=False)
+        a = a.reshape(-1)[np.sort(keep)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "latent.npy"), a)
+
+
 def run_k2(args):
     from kandinsky2 import ops
     from kandinsky2.model.gaussian_diffusion import FusedStep, create_ddpm_v22
@@ -386,6 +410,8 @@ def run_k2(args):
     sampler.start()
     ms = timed(one_step, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_latent(args.dump_outputs, x, world, rank)  # before the e2e steps below overwrite x from host memory
     ms_per_step = ms / args.steps
     value = world * 1e3 / ms_per_step
 
@@ -521,7 +547,11 @@ def main():
     ap.add_argument("--no-images", action="store_true", help="skip the whole-call images/s measurement")
     ap.add_argument("--no-configs", action="store_true", help="skip the other BASELINE configs' step geometries (N=1 only)")
     ap.add_argument("--inpaint", action="store_true", help="main workload = the inpainting UNet (9-channel stem)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the latents of the last timed step to DIR/latent.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "k2":
+        ap.error("--dump-outputs writes the outputs of the k2 step (--impl k2)")
     if args.impl == "reference":
         run_reference(args)
     elif args.impl == "torch_gpu":

@@ -77,7 +77,10 @@ __global__ void __launch_bounds__(256, 1) attention_d512_kernel(const __grid_con
   uint64_t* s_full = ring_empty + STAGES;  // 2
   uint64_t* p_full = s_full + 2;           // 1
   uint64_t* pv_done = p_full + 1;          // 1
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(pv_done + 1);
+  // the epilogue cannot wait for PV(nblk - 1) by pv_done's parity: the common path never waits for PV(j), so when the softmax
+  // of the last block ends, PV(nblk - 2) may still be pending, and its phase has the parity of the one the epilogue wants
+  uint64_t* o_full = pv_done + 1;          // 1: committed once, after the last PV product
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(o_full + 1);
 
   const int warp_idx = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -98,6 +101,7 @@ __global__ void __launch_bounds__(256, 1) attention_d512_kernel(const __grid_con
     }
     mbar_init(p_full, 4);
     mbar_init(pv_done, 1);
+    mbar_init(o_full, 1);
     fence_barrier_init();
   }
   if (warp_idx == 2) {
@@ -189,6 +193,7 @@ __global__ void __launch_bounds__(256, 1) attention_d512_kernel(const __grid_con
         }
         umma_commit(pv_done);
       }
+      umma_commit(o_full);
     }
   } else if (warp_idx >= 4) {
     // ===================================== softmax + epilogue =================================
@@ -274,7 +279,7 @@ __global__ void __launch_bounds__(256, 1) attention_d512_kernel(const __grid_con
       if (lane == 0) mbar_arrive(p_full);
     }
     // epilogue: O / l -> fp16, each thread writes the 256 channels of its row (512 contiguous bytes)
-    mbar_wait(pv_done, (nblk - 1) & 1);
+    mbar_wait(o_full, 0);
     tc_fence_after();
     const int q = q0 + row;
     const float inv = 1.f / l_run;

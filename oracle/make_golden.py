@@ -79,11 +79,20 @@ def golden_unet(name, cfg, B, H, W, ntext, wseed, iseed):
     print(f"{name}: reference out std {y_ref.std():.4f}, oracle-vs-reference max abs {err:.2e}")
 
 
+def golden_fp16_probe():
+    """The fp16 CPU arithmetic of the host that wrote the `out_ref_fp16` outputs above (unet_oracle.fp16_cpu_probe): a host
+    that reproduces it computes the reference's fp16 mode bit for bit like this one."""
+    probe = uo.fp16_cpu_probe()
+    torch.save(probe, os.path.join(GOLD, "fp16_cpu_probe.pt"))
+    print("fp16_cpu_probe:", probe["cpu_capability"])
+
+
 def main():
     os.makedirs(GOLD, exist_ok=True)
     torch.manual_seed(0)
     golden_unet("unet_tiny", uo.CONFIG_TINY, 2, 16, 16, 7, wseed=1, iseed=5)
     golden_unet("unet_tiny_inpaint", dict(uo.CONFIG_TINY, inpainting=True), 2, 16, 16, 7, wseed=2, iseed=6)
+    golden_fp16_probe()
     for extra in EXTRA:
         extra()
 

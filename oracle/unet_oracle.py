@@ -222,6 +222,28 @@ def to_reference_fp16(sd):
     return out
 
 
+def fp16_cpu_probe():
+    """Fingerprint of this host's fp16 CPU arithmetic: seeded fp16 conv2d / conv1d / bmm, GroupNorm and SiLU on fp16 data,
+    fp32 softmax, plus ATen's CPU capability.  oneDNN's fp16 kernels (AVX512-FP16 / AMX vs AVX512 / AVX2) and ATen's
+    vectorised kernels sum in different orders, so the fp16 mode's outputs differ between hosts by ~5e-3 at the tiny UNet's
+    size; hosts that agree on this probe bit for bit reproduce each other's fp16 forwards exactly.  Tensors are returned as
+    SHA-256 digests of their bytes."""
+    import hashlib
+    g = torch.Generator().manual_seed(0)
+    x = torch.randn(2, 64, 16, 16, generator=g).half()
+    w = (torch.randn(128, 64, 3, 3, generator=g) / 24).half()
+    b = torch.randn(128, generator=g).half()
+    w1 = (torch.randn(192, 128, 1, generator=g) / 11).half()
+    y = F.conv2d(x, w, b, padding=1)
+    q = F.conv1d(y.reshape(2, 128, 256), w1)
+    a = torch.bmm(q[:, :64].transpose(1, 2), q[:, 64:128])
+    n = F.group_norm(y.float(), 32).half()
+    out = dict(conv2d=y, conv1d=q, bmm=a, group_norm=n, silu=F.silu(n), softmax=torch.softmax(a.float() * 0.125, dim=-1).half())
+    out = {k: hashlib.sha256(v.contiguous().numpy().tobytes()).hexdigest() for k, v in out.items()}
+    out["cpu_capability"] = torch.backends.cpu.get_cpu_capability()
+    return out
+
+
 def unet_forward(sd, cfg, x, timesteps, full_emb=None, pooled_emb=None, image_emb=None, inpaint_image=None,
                  inpaint_mask=None, taps=None, fp16=False):
     """fp32 forward. `taps` (optional dict) receives intermediate activations keyed by block name.
