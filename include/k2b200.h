@@ -219,7 +219,8 @@ int k2_stem_im2col(const float* x, int Cx, const float* x2, int C2, const float*
  *   coef (device, fp32[8]): sqrt_recip_ac, sqrt_recipm1_ac, post_coef1, post_coef2, min_log, max_log,
  *   nonzero, sqrt(alphas_cumprod[next timestep]) (2.2 inpainting only).  cond_first: 1 = rows [0,B) conditional (2.1), 0 = unconditional first (2.2).
  *   threshold_mode 0: x0 = clamp(x0, -clip, clip); 1: additionally the reference's dynamic threshold
- *   s = max(percentile_99.5(|x0[sample 0]|), 1); x0 = clip(x0, -s, s)/s   (gaussian_diffusion.py:284-294).
+ *   s = max(percentile_99.5(|x0[sample 0]|), 1); x0 = clip(x0, -s, s)/s   (gaussian_diffusion.py:284-294), the percentile
+ *   bit-identical to np.percentile with numpy >= 2 semantics (float32 index, weight and interpolation).
  *   Split step for sharded runs (the reference's "sample 0" is GLOBAL sample 0): 2 = x0 + percentile of local sample 0 -> s in
  *   work[B*4*H*W], no update; 4 = x0 only; 3 = the update, with s read from work[B*4*H*W] (the caller broadcasts that float
  *   from the rank that owns global sample 0 between the two calls).

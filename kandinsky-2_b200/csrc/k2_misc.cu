@@ -277,8 +277,8 @@ __global__ void __launch_bounds__(256) sampler_x0_kernel(const SamplerParams p) 
 }
 
 // exact order statistics of |v[0..n)| (non-negative floats compare like their bit patterns):
-// 4-pass byte radix select, single block. Reproduces np.percentile(|x|, 99.5) with linear interpolation
-// (gaussian_diffusion.py:288-292) and s = max(s, 1).
+// 4-pass byte radix select, single block. Reproduces np.percentile(|x|, 99.5) with linear interpolation, numpy >= 2
+// semantics (gaussian_diffusion.py:288-292), and s = max(s, 1).
 __device__ float radix_select(const float* __restrict__ v, int n, int rank, unsigned int* hist, unsigned int* sh) {
   unsigned int prefix = 0, mask = 0;
   int k = rank;
@@ -315,17 +315,22 @@ __global__ void __launch_bounds__(1024) sampler_percentile_kernel(const float* _
   __shared__ unsigned int sh[2];
   pdl_wait();
   pdl_launch();
-  const double pos = 0.995 * static_cast<double>(n - 1);
-  int lo = static_cast<int>(floor(pos));
-  const double frac = pos - lo;
-  int hi = lo + 1 < n ? lo + 1 : n - 1;
+  // numpy >= 2 on float32 data stays in float32 (NEP 50; numpy/lib/_function_base_impl.py): percentile divides q by
+  // float32(100), the 'linear' virtual index is (n - 1) * q, _get_indexes takes floor / floor + 1 (both n - 1 when the index
+  // reaches n - 1), _get_gamma is the exact fraction, and _lerp rounds every operation to float32.  The _rn intrinsics keep
+  // nvcc from contracting any of these into an FMA.
+  const float q = __fdiv_rn(99.5f, 100.0f);
+  const float pos = __fmul_rn(static_cast<float>(n - 1), q);
+  const bool top = pos >= static_cast<float>(n - 1);
+  const int lo = top ? n - 1 : static_cast<int>(floorf(pos));
+  const int hi = top ? n - 1 : lo + 1;
   const float a = radix_select(x0, n, lo, hist, sh);
   const float b = radix_select(x0, n, hi, hist, sh);
   if (threadIdx.x == 0) {
     // numpy _lerp: a + (b-a)*t, switched to b - (b-a)*(1-t) for t >= 0.5
-    const double da = a, db = b;
-    double r = (frac >= 0.5) ? db - (db - da) * (1.0 - frac) : da + (db - da) * frac;
-    float s = static_cast<float>(r);
+    const float t = __fsub_rn(pos, static_cast<float>(lo));
+    const float d = __fsub_rn(b, a);
+    const float s = (t >= 0.5f) ? __fsub_rn(b, __fmul_rn(d, __fsub_rn(1.0f, t))) : __fadd_rn(a, __fmul_rn(d, t));
     *sval = fmaxf(s, 1.0f);
   }
 }

@@ -9,8 +9,8 @@ Replaces, for the hot path (SURVEY.md 8a rows a9-a11):
 The reference runs ~30 elementwise launches, an H2D copy per table lookup and a D2H sync (np.percentile)
 per step; here one step is [UNet forward graph] + k2_sampler_step (2-3 launches, no host sync): the
 per-step scalars come from a device table, the 99.5-percentile dynamic threshold is an exact radix select
-on the device.  Only learned-range variance / epsilon prediction (the Kandinsky decoder configuration,
-configs.py:150-162) is implemented.
+on the device with np.percentile's interpolation, numpy >= 2 semantics.  Only learned-range variance /
+epsilon prediction (the Kandinsky decoder configuration, configs.py:150-162) is implemented.
 """
 import numpy as np
 import torch
